@@ -18,7 +18,7 @@ separately on the device and reported with their roofline fractions (`roofline` 
 launches for this batch -- named in `roofline.kernel` --, HBM; `roofline_vit`).  Every generate call passes eos_token_id=None: exactly
 `--new-tokens` decode steps run on every path.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--model valley-13b|valley2-7b|tiny] ...
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--model valley-13b|valley2-7b|tiny] [--dump-outputs DIR] ...
   N>1: python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 --impl reference: the reference algorithm's CPU path (oracle/valley_oracle.py -- plain PyTorch CPU ops, the ATen kernels the
@@ -130,6 +130,35 @@ def decode_bytes_per_step(spec, B, S):
     w = 2 * (L * (4 * H * H + 3 * H * I) + V * H)
     kv = B * S * 2 * L * H * 2 + B * 2 * L * H * 2
     return w + kv
+
+
+def gather_rows(x, world):
+    """every rank's rows of ``x`` (equal shapes), in rank order: the whole batch on every rank"""
+    if world == 1:
+        return x
+    import torch.distributed as dist
+    parts = [torch.empty_like(x) for _ in range(world)]
+    dist.all_gather(parts, x.contiguous())
+    return torch.cat(parts)
+
+
+DUMP_CAP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays, rank=0):
+    """rank 0 writes each tensor as out_dir/<name>.npy in float64; an array past DUMP_CAP_BYTES is cut to a fixed, seeded
+    sample of its rows so that all files together stay under the cap"""
+    if rank != 0:
+        return
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    budget = DUMP_CAP_BYTES // max(len(arrays), 1)
+    for name, x in arrays.items():
+        x = x.detach().cpu().double().numpy()
+        if x.nbytes > budget:
+            keep = max(1, budget // max(x[0].nbytes, 1))
+            x = x[np.sort(np.random.default_rng(0).choice(len(x), keep, replace=False))]
+        np.save(os.path.join(out_dir, f"{name}.npy"), x)
 
 
 class ClockSampler:
@@ -334,7 +363,14 @@ def main():
     ap.add_argument("--no-7b", action="store_true", help="skip the extra valley2-7b B=1 figures (BASELINE config 2)")
     ap.add_argument("--vit-sweep", action="store_true", help="also time ViT encode over F (BASELINE config 5); N > 1: strong scaling, F fixed")
     ap.add_argument("--gpu-eager-baseline", action="store_true", help="also time the oracle as eager torch-CUDA ops on the GPU (SURVEY 8d)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned (the generated token ids of every "
+                         "sequence) to DIR/<name>.npy as float64, for comparing two builds output for output")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     spec = syn.SPECS[a.model]
     rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
     local = int(os.environ.get("LOCAL_RANK", 0))
@@ -490,6 +526,8 @@ def main():
         clk.start()
     ms_step, launches, toks = timed(step_device, a.steps, max(a.warmup, 3))
     clocks = clk.stop() if rank == 0 else None
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, {"tokens": gather_rows(toks, world)}, rank)
     ms_e2e, _, toks_e2e = timed(step_e2e, a.steps, 1)
 
     # ---- the two halves of the metric, timed separately on the device ----

@@ -251,9 +251,10 @@ def main():
                 spec=spec.name, seed=seed, B=B, T=T,
                 vit_hidden_m2_sub=hs[-2][:, ::4, ::8].clone(), vit_hidden_m1_sub=hs[-1][:, ::4, ::8].clone(),
                 prefill_logits_last=out.logits[:, -1, :].clone(), prefill_logits_sub=out.logits[:, ::16, ::8].clone(),
-                greedy_tokens=r_tok, greedy_logits=r_log, splice=gold_splice, errors=errs, leftpad=gold_leftpad, loss=gold_loss,
+                greedy_tokens=r_tok, greedy_logits=r_log, errors=errs, leftpad=gold_leftpad, loss=gold_loss,
             ), os.path.join(GOLD, f"ref_{spec.name}.pt"))
-            print("  wrote", f"tests/golden/ref_{spec.name}.pt")
+            torch.save(gold_splice, os.path.join(GOLD, f"ref_{spec.name}_splice.pt"))       # own file: every fixture stays under 1 MB
+            print("  wrote", f"tests/golden/ref_{spec.name}.pt", f"tests/golden/ref_{spec.name}_splice.pt")
         # --- pooling variants (valley_model.py:205-213): max, temporal_importance (v2), temporal_transformer (v3) -------
         import transformers
         for spec in (syn.TINY_MAX, syn.TINY_V2, syn.TINY_V3):
@@ -283,7 +284,7 @@ def main():
             assert (plain - grabbed["e"]).abs().max() > 1e-3          # the variant really differs from mean pooling
             close(O.causal_lm_forward(sd, cfg, tok, ids, px, None), out.logits, "prefill logits")
             p0 = (ids[0] == tok.im_start_token).nonzero()[0, 0] + 1
-            torch.save(dict(spec=spec.name, seed=seed, B=B, T=T, pooled_rows=grabbed["e"][:, p0:p0 + 256, :].clone()[:, ::4, ::4],
+            torch.save(dict(spec=spec.name, seed=seed, B=B, T=T, pooled_rows=grabbed["e"][:, p0:p0 + 256, ::4][:, ::4].clone(),
                             embeds_sub=grabbed["e"][:, :, ::8].clone(), prefill_logits_last=out.logits[:, -1, :].clone()),
                        os.path.join(GOLD, f"ref_{spec.name}.pt"))
             print("  wrote", f"tests/golden/ref_{spec.name}.pt")

@@ -316,6 +316,9 @@ def test_splice_plan_and_oracle_match_the_reference_on_fuzzed_rows():
     tok, lib = Hh.oracle_tok(spec), _lib.load()
     seen = {}
     for i, (row, (kind, val)) in enumerate(zip(g["rows"], g["results"])):
+        row = row.long()                                             # stored as int16 to keep the fixture small
+        if kind == "map":
+            val = val.int()
         seen[kind] = seen.get(kind, 0) + 1
         code, smap, iidx = plan(row[None], T, vly_tokens(spec))
         if kind == "plain":

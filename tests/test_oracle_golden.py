@@ -36,12 +36,13 @@ def test_oracle_matches_reference_fixture(name):
 @pytest.mark.parametrize("name", ["tiny"])
 def test_oracle_splice_cases_match_reference(name):
     g = torch.load(os.path.join(GOLD, f"ref_{name}.pt"))
+    splice = torch.load(os.path.join(GOLD, f"ref_{name}_splice.pt"))
     spec = syn.SPECS[name]
     sd = syn.make_state_dict(spec, g["seed"])
     cfg, tok = Hh.oracle_cfg(spec), Hh.oracle_tok(spec)
     px = syn.make_pixels(g["B"], g["T"], g["seed"])
     with torch.no_grad():
-        for case, d in g["splice"].items():
+        for case, d in splice.items():
             if isinstance(d["n_frames"], list):          # images given as a list of clips with different frame counts
                 cpx = [px[i, :n] for i, n in enumerate(d["n_frames"])]
             else:
